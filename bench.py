@@ -5,6 +5,7 @@
     torchrun --nproc-per-node N ... bench.py --gpus N ...       # weak scaling: 16384 envs per rank (--scaling strong: 16384 in total)
     python bench.py --impl reference ...                        # CPU port of the path (oracle/), host cores, same config
     python bench.py --workload humanoid|anymal|shadow_hand|cartpole
+    python bench.py ... --dump-outputs DIR                      # also write what the last timed step returned, DIR/<name>.npy
 
 One "step" = one VecTask.step() over all envs under random actions U(-1,1) (the README rollout loop of the reference,
 README.md:39-51).  `value` is measured THROUGH `env.step(actions)` (the reference's metric, tasks/base/vec_task.py:360-408);
@@ -326,9 +327,7 @@ def run_reference_arm(args):
     task, n_full, _ = WORKLOADS[args.workload]
     n = args.num_envs or n_full
     cores = os.cpu_count() or 1
-    # each step is the whole workload; K bounded so the run ends within a few minutes whatever the driver asks for
-    est = {"Ant": 0.8e6, "Humanoid": 0.25e6, "Cartpole": 4e6, "AnymalTerrain": 0.15e6, "ShadowHand": 0.3e6}[task] * cores / 128.0
-    k = max(3, min(args.steps, int(60.0 * est / n)))
+    k = args.steps                                          # each step is the whole workload
     v, secs = cpu_pipeline(task, n, k, cores, warmup=max(1, min(args.warmup, 3)))
     line = {"metric": METRIC, "impl": "reference", "value": v, "unit": "env-steps/s", "n_gpus": args.gpus,
             "steps": k, "warmup": args.warmup, "ms_per_step": 1e3 * secs / k,
@@ -342,6 +341,35 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------ GPU arm
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def step_outputs(result):
+    """What VecTask.step() hands its caller (obs dict, reward, reset, the tensors in extras) as float32 / float64 host arrays."""
+    import torch
+    obs_dict, rew, reset, extras = result
+    named = dict(obs_dict)
+    named.update(rew=rew, reset=reset)
+    named.update({k: v for k, v in extras.items() if torch.is_tensor(v)})
+    return {k: (v.double() if v.dtype == torch.float64 else v.float()).cpu().numpy() for k, v in named.items()}
+
+
+def dump_outputs(outputs, out_dir):
+    """Writes out_dir/<name>.npy.  Above DUMP_LIMIT_BYTES in all, every per-env array keeps the same fixed, seeded sample of
+    envs, whose indices go to sample_envs.npy."""
+    n = outputs["rew"].shape[0]
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        per_env = sum(a.nbytes for a in outputs.values() if a.ndim and a.shape[0] == n) / n
+        keep = int((DUMP_LIMIT_BYTES - (total - per_env * n) - 8 * n) // per_env)
+        rows = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        outputs = {k: (a[rows] if a.ndim and a.shape[0] == n else a) for k, a in outputs.items()}
+        outputs["sample_envs"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_gpu_arm(args):
     import torch
     import torch.distributed as dist
@@ -386,12 +414,14 @@ def run_gpu_arm(args):
     w0 = time.perf_counter()
     t0.record()
     for k in range(args.steps):
-        envs[k % R].step(ring[k % 16])
+        last = envs[k % R].step(ring[k % 16])
     t1.record()
     host_issue_s = time.perf_counter() - w0                 # host time to ISSUE the K steps (no sync inside)
     barrier()
     launches = sum(e_.sim.launch_count() for e_ in envs) - l0
     total_ms = t0.elapsed_time(t1)
+    # the env buffers are stepped again below: copy the last timed step's results out now
+    outputs = step_outputs(last) if args.dump_outputs else None
     # ---- device only: the same K steps as bare C-ABI launches (b2g_task_step), same rotation: the kernel time
     d0, d1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
@@ -521,6 +551,8 @@ def run_gpu_arm(args):
         v, secs = cpu_pipeline(task, n, ks, cores)
         line["cpu_baseline"] = {"value": v, "unit": "env-steps/s", "cores": cores, "kind": "port",
                                 "sample": f"{n} envs x {ks} control steps, {secs:.1f} s ({CPU_WHAT})"}
+    if outputs is not None:
+        dump_outputs(outputs, args.dump_outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -539,7 +571,13 @@ def main():
     ap.add_argument("--sets", type=int, default=0, help="independent env sets stepped round-robin (0 = enough to exceed 1.5 x L2)")
     ap.add_argument("--no-rollout", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed VecTask.step() returned as DIR/<name>.npy (same arguments, same inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none to give")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -137,8 +137,7 @@ def test_unmodified_reference_shadow_hand_runs_on_the_shim(compat_cpu):
     assert "consecutive_successes" in extras and "time_outs" in extras
 
 
-@needs_reference
-def test_procedural_primitive_assets_become_the_free_object(compat_cpu):
+def test_procedural_primitive_assets_become_the_free_object(compat_cpu, reference_assets):
     """gym.create_sphere / create_box / create_capsule (ball_balance.py:277, franka_cube_stack.py:223-245): one primitive, mass =
     density x volume, and as the second actor of an env the engine's rounded box (sphere: a point + radius)."""
     from isaacgym import gymapi
@@ -157,7 +156,7 @@ def test_procedural_primitive_assets_become_the_free_object(compat_cpu):
     assert abs(float(cap.model.mass[0]) - 200.0 * (math.pi * 0.05 ** 2 * 0.4 + 4 / 3 * math.pi * 0.05 ** 3)) < 1e-9
     # the ball as the free object of a two-actor env (articulation + ball): cartpole stands in for the articulation
     copt = gymapi.AssetOptions(); copt.fix_base_link = True; copt.angular_damping = 0.5
-    cart = gym.load_asset(sim, os.path.join(REFERENCE, "assets"), "urdf/cartpole.urdf", copt)
+    cart = gym.load_asset(sim, reference_assets, "urdf/cartpole.urdf", copt)
     for i in range(2):
         e = gym.create_env(sim, gymapi.Vec3(-1, -1, 0), gymapi.Vec3(1, 1, 1), 2)
         gym.create_actor(e, cart, gymapi.Transform(gymapi.Vec3(0, 0, 2.0)), "cartpole", i, 1, 0)
@@ -170,16 +169,22 @@ def test_procedural_primitive_assets_become_the_free_object(compat_cpu):
     assert torch.allclose(rs[:, 1, 0:3], torch.tensor([0.5, 0.0, 1.0]))
 
 
-@needs_reference
-def test_name_maps_and_small_accessors_of_the_shim(compat_cpu):
+def test_name_maps_and_small_accessors_of_the_shim(compat_cpu, reference_assets):
     """the dictionary / count accessors other reference tasks use around the tensor API (franka_cube_stack.py:391, allegro_hand.py,
-    ant.py:307-321 debug lines): body / DOF order = the tensors' order"""
-    import importlib
-    mod = importlib.import_module("isaacgymenvs.tasks.ant")
+    ant.py:307-321 debug lines): body / DOF order = the tensors' order.  The scene is the one ant.py builds: one Ant per env."""
+    from isaacgym import gymapi
+    gym = gymapi.acquire_gym()
+    sp = gymapi.SimParams(); sp.dt, sp.substeps = 0.0166, 2
+    sim = gym.create_sim(0, -1, gymapi.SIM_PHYSX, sp)
+    gym.add_ground(sim, gymapi.PlaneParams())
+    ant = gym.load_asset(sim, reference_assets, "mjcf/nv_ant.xml", gymapi.AssetOptions())
     n = 4
-    env = mod.Ant(cfg=_cfg("Ant", n), rl_device="cpu", sim_device="cpu", graphics_device_id=-1, headless=True,
-                  virtual_screen_capture=False, force_render=False)
-    gym, sim, e0 = env.gym, env.sim, env.envs[0]
+    envs = []
+    for i in range(n):
+        envs.append(gym.create_env(sim, gymapi.Vec3(-2, -2, 0), gymapi.Vec3(2, 2, 2), 2))
+        gym.create_actor(envs[i], ant, gymapi.Transform(gymapi.Vec3(0, 0, 0.44)), "ant", i, 1, 0)
+    gym.prepare_sim(sim)
+    e0 = envs[0]
     bd, dd = gym.get_actor_rigid_body_dict(e0, 0), gym.get_actor_dof_dict(e0, 0)
     assert len(bd) == 9 and len(dd) == 8 and bd["torso"] == 0 and sorted(dd.values()) == list(range(8))
     assert gym.get_actor_rigid_body_names(e0, 0)[bd["front_left_foot"]] == "front_left_foot"

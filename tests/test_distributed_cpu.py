@@ -61,7 +61,7 @@ def test_hand_resets_do_not_depend_on_the_sharding():
     gold = np.load(_os.path.join(_os.path.dirname(_os.path.abspath(__file__)), "golden", "shadow_hand.npz"))
     st, P, actions = golden_case(gold, "a")
     n = 16
-    cut = lambda d, sl: {k: (v[sl].copy() if isinstance(v, np.ndarray) and v.shape[:1] == (256,) else v) for k, v in d.items()}
+    cut = lambda d, sl: {k: (v[sl].copy() if isinstance(v, np.ndarray) and v.shape[:1] == actions.shape[:1] else v) for k, v in d.items()}
     whole, Pw = cut(st, slice(0, n)), cut(P, slice(0, n))
     whole["reset"][:] = 1
     T.hand_pre_physics(whole, actions[:n], dict(Pw, env_id_offset=0))

@@ -136,7 +136,7 @@ def test_loco_baseline_sizes_and_tail_lanes(task, n):
     _loco_check(env, _loco_orc(env, threads=16), task, 3, rng)
 
 
-def test_quad_path_equals_generic_path():
+def test_quad_path_equals_generic_path(tmp_path):
     """The specialised Ant step (b2g_quad.cuh) and the generic slot-program Stepper are two formulations of one
     sub-step: from identical states and actions, a whole control step agrees to fp32 round-off."""
     code = r'''
@@ -157,7 +157,7 @@ np.savez(sys.argv[1], obs=obs["obs"].cpu().numpy(), rew=rew.cpu().numpy(), reset
 ''' % ROOT
     res = []
     for noquad in ("0", "1"):
-        out = os.path.join("/tmp", f"b2g_quadcmp_{noquad}.npz")
+        out = str(tmp_path / f"quadcmp_{noquad}.npz")
         env_ = dict(os.environ, B2G_NO_QUAD=noquad)
         subprocess.check_call([sys.executable, "-c", code, out], env=env_, cwd=ROOT)
         res.append(dict(np.load(out)))
@@ -287,7 +287,7 @@ def test_hand_baseline_size_simulate_matches_oracle():
 
 
 # ------------------------------------------------------------------------------------ fast trigonometry
-def test_fast_trig_build_is_bounded_against_exact_trig_build():
+def test_fast_trig_build_is_bounded_against_exact_trig_build(tmp_path):
     """The product build evaluates joint rotations with __sincosf (B2G_FAST_TRIG=1).  Same library built with sincosf:
     one control step from states that include joint angles AT and beyond the limits (|q| up to 2.8 rad for the
     Humanoid knee) differs by < 2e-5 in base pose, < 1e-4 in joint positions (90 % below 1e-5, median below 1e-6) and < 5e-3 relative in joint velocities; after 30-step
@@ -331,7 +331,7 @@ np.savez(sys.argv[1], **out)
 ''' % ROOT
     res = []
     for lib in ("", exact):
-        out = os.path.join("/tmp", f"b2g_trig_{int(bool(lib))}.npz")
+        out = str(tmp_path / f"trig_{int(bool(lib))}.npz")
         env_ = dict(os.environ)
         if lib:
             env_["B2G_LIB"] = lib

@@ -7,7 +7,7 @@ import re
 import numpy as np
 import pytest
 
-from tests.conftest import needs_reference, REFERENCE, ROOT
+from tests.conftest import REFERENCE, ROOT
 
 
 def test_library_builds_and_exports_the_declared_abi():
@@ -47,11 +47,14 @@ def test_no_cpu_fallback():
         engine.Sim(load_compiled("ant"), 4, 0.0166, 2, device="cpu")
 
 
-@needs_reference
 @pytest.mark.parametrize("task", ["Cartpole", "Ant", "Humanoid", "ShadowHand"])
-def test_reference_yaml_loads_unmodified_and_matches_builtin(task):
+def test_reference_yaml_loads_unmodified_and_matches_builtin(task, reference_cfg):
+    """The built-in config against the reference's YAML as load_reference_cfg composes it (tests/golden/reference_cfg.json;
+    where a reference checkout is present, also against a fresh load of its YAML)."""
     from isaacgymenvs_b200 import config
-    ref = config.load_reference_cfg(os.path.join(REFERENCE, "isaacgymenvs", "cfg"), task, {"num_envs": 64})
+    ref = {"task": reference_cfg["task_cfg_num_envs_64"][task]}
+    if os.path.isdir(REFERENCE):
+        assert config.load_reference_cfg(os.path.join(REFERENCE, "isaacgymenvs", "cfg"), task, {"num_envs": 64})["task"] == ref["task"]
     own = config.builtin_cfg(task, {"num_envs": 64})
 
     def cmp(a, b, path=""):
@@ -66,29 +69,29 @@ def test_reference_yaml_loads_unmodified_and_matches_builtin(task):
     assert ref["task"]["sim"]["physx"]["num_threads"] == 4
 
 
-@needs_reference
-def test_importer_known_answers_and_compiled_blobs_are_current():
-    """SURVEY.md 8c importer known-answers (analytic, from the XML) + committed blobs == fresh import."""
+def test_importer_known_answers_and_compiled_blobs_are_current(reference_assets):
+    """SURVEY.md 8c importer known-answers (analytic, from the XML) + committed blobs == fresh import of the reference's
+    robot descriptions (tests/golden/reference_assets.tar.xz)."""
     from isaacgymenvs_b200.importer.mjcf import load_mjcf
     from isaacgymenvs_b200.importer.urdf import load_urdf
     from isaacgymenvs_b200.importer.model import BuildOptions
     from isaacgymenvs_b200.assets import load_compiled
     from isaacgymenvs_b200.assets.compile_assets import SPECS
-    ant = load_mjcf(os.path.join(REFERENCE, "assets/mjcf/nv_ant.xml"))
+    ant = load_mjcf(os.path.join(reference_assets, "mjcf/nv_ant.xml"))
     assert abs(ant.mass[0] - 0.48388) < 1e-5 and abs(ant.mass[1] - 0.039158) < 1e-6 and abs(ant.mass[2] - 0.067592) < 1e-6
     assert abs(ant.total_mass() - 0.91088) < 1e-5
     assert ant.dof_names == ["hip_1", "ankle_1", "hip_2", "ankle_2", "hip_3", "ankle_3", "hip_4", "ankle_4"]
     assert np.allclose(np.degrees(ant.lower[1:3]), [-40, 30]) and np.allclose(ant.armature[1:], 0.01) and np.allclose(ant.damping[1:], 0.1)
-    hum = load_mjcf(os.path.join(REFERENCE, "assets/mjcf/nv_humanoid.xml"))
+    hum = load_mjcf(os.path.join(reference_assets, "mjcf/nv_humanoid.xml"))
     assert hum.nb == 16 and hum.ndof == 21 and hum.dof_names[:3] == ["abdomen_z", "abdomen_y", "abdomen_x"]
     assert hum.actuator_joint[:2] == ["abdomen_y", "abdomen_z"]
-    cp = load_urdf(os.path.join(REFERENCE, "assets/urdf/cartpole.urdf"), BuildOptions(fix_base_link=True))
+    cp = load_urdf(os.path.join(reference_assets, "urdf/cartpole.urdf"), BuildOptions(fix_base_link=True))
     assert cp.ndof == 2 and cp.jtype[1] == 1 and cp.jtype[2] == 0 and cp.limited[2] == 0 and abs(cp.lpos[2][0] - 0.12) < 1e-12
-    any_ = load_urdf(os.path.join(REFERENCE, "assets/urdf/anymal_c/urdf/anymal_minimal.urdf"),
+    any_ = load_urdf(os.path.join(reference_assets, "urdf/anymal_c/urdf/anymal_minimal.urdf"),
                      BuildOptions(collapse_fixed_joints=True, replace_cylinder_with_capsule=True))
     assert any_.nb == 13 and any_.ndof == 12 and len(any_.geom_type) == 9      # base + 4 x (knee, shank) ... feet
     for name, (rel, opts) in SPECS.items():
-        path = os.path.join(REFERENCE, "assets", rel)
+        path = os.path.join(reference_assets, rel)
         fresh = load_urdf(path, opts, name=name) if rel.endswith(".urdf") else load_mjcf(path, opts, name=name)
         blob = load_compiled(name)
         for f in ("parent", "jtype", "axis", "lpos", "mass", "com", "inertia", "lower", "upper", "cp_pos", "cp_radius", "limit_k"):
@@ -176,6 +179,52 @@ def test_bench_reference_arm_prints_the_contract_line(workload):
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["vs_baseline"] is None and "workload" in d["config"]
+
+
+def test_bench_dump_outputs_writes_what_step_returned(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one float32 / float64 .npy per array VecTask.step() returns; above the size limit every per-env
+    array keeps the same seeded sample of envs, whose indices are written beside them."""
+    import importlib.util, torch
+    spec = importlib.util.spec_from_file_location("b2g_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec); spec.loader.exec_module(bench)
+    n = 1000
+    g = torch.Generator().manual_seed(1)
+    result = ({"obs": torch.rand(n, 60, generator=g)}, torch.rand(n, generator=g, dtype=torch.float64), torch.randint(0, 2, (n,), generator=g),
+              {"time_outs": torch.rand(n, generator=g) > 0.5, "consecutive_successes": torch.tensor(1.5), "episode": 3})
+    outs = bench.step_outputs(result)
+    assert sorted(outs) == ["consecutive_successes", "obs", "reset", "rew", "time_outs"]
+    assert outs["rew"].dtype == np.float64 and all(outs[k].dtype == np.float32 for k in ("obs", "reset", "time_outs", "consecutive_successes"))
+    assert np.array_equal(outs["reset"], result[2].numpy()) and np.array_equal(outs["obs"], result[0]["obs"].numpy())
+    bench.dump_outputs(outs, str(tmp_path / "whole"))
+    for k, a in outs.items():
+        assert np.array_equal(np.load(tmp_path / "whole" / f"{k}.npy"), a)
+    assert not (tmp_path / "whole" / "sample_envs.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 100_000)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(dict(outs), str(tmp_path / d))
+    got = {k: np.load(tmp_path / "s1" / f"{k}.npy") for k in list(outs) + ["sample_envs"]}
+    rows = got["sample_envs"].astype(np.int64)
+    assert got["sample_envs"].dtype == np.float64 and 0 < len(rows) < n and sum(a.nbytes for a in got.values()) <= 100_000
+    for k in ("obs", "rew", "reset", "time_outs"):
+        assert np.array_equal(got[k], outs[k][rows])
+        assert np.array_equal(np.load(tmp_path / "s2" / f"{k}.npy"), got[k])
+    assert got["consecutive_successes"] == np.float32(1.5)
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_of_the_gpu_path(tmp_path):
+    """`bench.py --dump-outputs DIR` on the GPU: the last timed step's observation / reward / reset / time-out arrays land in DIR
+    and the JSON line reports the requested step count."""
+    import json, subprocess, sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "1", "--num-envs", "512",
+                          "--sets", "2", "--no-cpu-baseline", "--no-rollout", "--dump-outputs", str(tmp_path / "out")],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])
+    assert d["steps"] == 3
+    got = {f[:-4]: np.load(tmp_path / "out" / f) for f in os.listdir(tmp_path / "out")}
+    assert {"obs", "rew", "reset", "time_outs"} <= set(got) and got["obs"].shape == (512, 60) and got["rew"].shape == (512,)
+    assert all(a.dtype in (np.float32, np.float64) and np.isfinite(a).all() for a in got.values())
 
 
 def test_bench_reference_arm_other_ranks_exit_quietly():
@@ -301,20 +350,19 @@ def test_train_launcher_maps_reference_overrides():
             tr.to_ppo_argv(tr.parse_overrides(bad))
 
 
-@needs_reference
-def test_train_launcher_hyperparameters_are_the_reference_yaml():
-    import importlib.util, yaml
+def test_train_launcher_hyperparameters_are_the_reference_yaml(reference_cfg):
+    """train.py's PPO table against the values of the reference's train / task YAML (tests/golden/reference_cfg.json)."""
+    import importlib.util
     spec = importlib.util.spec_from_file_location("b2g_train", os.path.join(ROOT, "train.py"))
     tr = importlib.util.module_from_spec(spec); spec.loader.exec_module(tr)
+    assert sorted(reference_cfg["ppo"]) == sorted(tr.PPO)
     for task, hp in tr.PPO.items():
-        d = yaml.safe_load(open(os.path.join(REFERENCE, "isaacgymenvs", "cfg", "train", task + "PPO.yaml")))
-        c, n = d["params"]["config"], d["params"]["network"]
-        assert n["mlp"]["units"] == hp["units"] and float(c["learning_rate"]) == hp["lr"] and c["horizon_length"] == hp["horizon"]
+        c = reference_cfg["ppo"][task]
+        assert c["units"] == hp["units"] and float(c["learning_rate"]) == hp["lr"] and c["horizon_length"] == hp["horizon"]
         assert c["minibatch_size"] == hp["minibatch"] and c["mini_epochs"] == hp["mini_epochs"] and c["critic_coef"] == hp["critic_coef"]
-        assert c["kl_threshold"] == hp["kl"] and c["reward_shaper"]["scale_value"] == hp["rew_scale"] and float(c["bounds_loss_coef"]) == hp["bounds"]
+        assert c["kl_threshold"] == hp["kl"] and c["scale_value"] == hp["rew_scale"] and float(c["bounds_loss_coef"]) == hp["bounds"]
         assert str(hp["epochs"]) in c["max_epochs"] and c["gamma"] == 0.99 and c["tau"] == 0.95 and c["e_clip"] == 0.2
-        t = yaml.safe_load(open(os.path.join(REFERENCE, "isaacgymenvs", "cfg", "task", task + ".yaml")))
-        assert str(hp["num_envs"]) in str(t["env"]["numEnvs"])
+        assert str(hp["num_envs"]) in c["num_envs"]
 
 
 # ---------------------------------------------------------------------------------------------
@@ -344,8 +392,7 @@ def test_mesh_mass_properties_are_those_of_the_enclosed_solid(tmp_path):
         mass_properties(np.zeros((3, 3)), np.array([[0, 1, 2]]))
 
 
-@needs_reference
-def test_franka_links_get_their_mass_from_the_collision_meshes():
+def test_franka_links_get_their_mass_from_the_collision_meshes(reference_assets):
     """franka_panda_gripper.urdf has no <inertial>: density x mesh volume (AssetOptions.density 1000) must give a ~20 kg arm, and
     the skipped mesh CONTACT is announced, not silent."""
     import warnings
@@ -353,7 +400,7 @@ def test_franka_links_get_their_mass_from_the_collision_meshes():
     from isaacgymenvs_b200.importer.model import BuildOptions, UnmodelledGeometryWarning
     with warnings.catch_warnings(record=True) as w:
         warnings.simplefilter("always")
-        m = load_urdf(os.path.join(REFERENCE, "assets/urdf/franka_description/robots/franka_panda_gripper.urdf"), BuildOptions(fix_base_link=True))
+        m = load_urdf(os.path.join(reference_assets, "urdf/franka_description/robots/franka_panda_gripper.urdf"), BuildOptions(fix_base_link=True))
     assert sum(issubclass(x.category, UnmodelledGeometryWarning) for x in w) == 1
     assert 15.0 < m.total_mass() < 25.0 and (m.mass[:8] > 1.0).all() and (m.inertia[1:8, :3] > 1e-3).all()
     assert m.body_joint_names[8] == "panda_hand_joint" and m.body_names[8] == "panda_hand" and m.ndof == 9

@@ -285,11 +285,7 @@ def test_mass_matrix_is_the_inertia_the_aba_step_inverts(name):
 
 # ---------------------------------------------------------------------------------------------------------------
 # the reference's indexing idiom for the operational-space controller (franka_cube_stack.py:388-394, 600-627) on the Franka itself
-from tests.conftest import needs_reference, REFERENCE
-
-
-@needs_reference
-def test_franka_jacobian_is_indexed_by_joint_as_the_reference_does():
+def test_franka_jacobian_is_indexed_by_joint_as_the_reference_does(reference_assets):
     """`hand_joint_index = gym.get_actor_joint_dict(env, franka)['panda_hand_joint']; j_eef = jacobian[:, hand_joint_index, :, :7]`:
     with one joint per non-root body the joint index addresses the hand body's row of the fixed-base Jacobian.  Checked on the
     Franka URDF (mesh collisions skipped with a warning: kinematics and inertias come from <inertial>): J_eef qd = the hand
@@ -300,7 +296,7 @@ def test_franka_jacobian_is_indexed_by_joint_as_the_reference_does():
     from isaacgymenvs_b200.compat import gymapi
     with warnings.catch_warnings(record=True) as w:
         warnings.simplefilter("always")
-        m = load_urdf(os.path.join(REFERENCE, "assets/urdf/franka_description/robots/franka_panda_gripper.urdf"), BuildOptions(fix_base_link=True))
+        m = load_urdf(os.path.join(reference_assets, "urdf/franka_description/robots/franka_panda_gripper.urdf"), BuildOptions(fix_base_link=True))
     assert any(issubclass(x.category, UnmodelledGeometryWarning) for x in w) and len(m.unmodelled_geoms) == 11
     gym = gymapi.acquire_gym()
     asset = gymapi._Asset(m, gymapi.AssetOptions())
